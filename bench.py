@@ -17,17 +17,26 @@ one polynomial is taken through lagrange_to_coeff -> coeff_to_extended -> extend
 Horner evaluations at domain points.  A mismatch exits with status 3 and prints no JSON line.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config 1..5] [--sweep 1,2,4,5|none]
+                    [--dump-outputs DIR]
+
+`--steps` is the number of timed steps of each step timing of the headline config (resident step in both transform
+placements, resident proof, host-buffer step); the per-op timings take 3 repetitions and the sweep extras 2-3 steps each.
+`--dump-outputs DIR` writes what the last timed resident step computed to DIR/<name>.npy (see `Workload.outputs`).
 """
 from __future__ import annotations
 import argparse
+import atexit
 import json
 import math
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
+sys.dont_write_bytecode = True  # the tree may be read-only: nothing is cached next to the sources
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -215,6 +224,49 @@ def horner_mont(coeff_limbs: np.ndarray, x: int) -> int:
     return acc * MONT_RINV_R % R_MOD
 
 
+# ------------------------------------------------------------------------------------------------ --dump-outputs
+# Outputs are written as canonical integers (out of Montgomery form, points in affine form), so that two builds that
+# represent the same values differently still compare equal.  Each 256-bit value is 8 little-endian 32-bit limbs, held
+# exactly in float64.
+DUMP_ROWS = 8192         # rows per column / polynomial: a fixed, seeded sample of the longer ones
+DUMP_LIMIT = 64 << 20    # bytes in all (config 4, the widest schedule, writes about 32 MB)
+
+
+def dump_rows(n: int) -> np.ndarray:
+    """the sorted row indices written for an output of n rows (the same on every run)"""
+    if n <= DUMP_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0xD0D0).choice(n, DUMP_ROWS, replace=False))
+
+
+def ints_to_limbs32(vals) -> np.ndarray:
+    return np.frombuffer(b"".join(v.to_bytes(32, "little") for v in vals), dtype=np.uint32).astype(np.float64).reshape(-1, 8)
+
+
+def fr_canonical(mont_limbs: np.ndarray) -> np.ndarray:
+    """Montgomery Fr elements (m x 4 u64) -> their values, m x 8 limbs"""
+    buf = np.ascontiguousarray(mont_limbs, dtype=np.uint64).tobytes()
+    return ints_to_limbs32([int.from_bytes(buf[i:i + 32], "little") * MONT_RINV_R % R_MOD for i in range(0, len(buf), 32)])
+
+
+def g1_affine(xyz_limbs) -> np.ndarray:
+    """one G1 point as the library returns it (12 u64, Jacobian, Montgomery) -> affine (x, y), 16 limbs; the identity
+    is all zeros ((0, 0) is not on the curve)"""
+    X, Y, Z = (limbs_to_int(r) * MONT_RINV_P % P_MOD for r in np.asarray(xyz_limbs, dtype=np.uint64).reshape(3, 4))
+    if Z == 0:
+        return ints_to_limbs32([0, 0]).reshape(16)
+    zi = pow(Z, -1, P_MOD)
+    return ints_to_limbs32([X * zi * zi % P_MOD, Y * zi * zi * zi % P_MOD]).reshape(16)
+
+
+def write_outputs(outputs: dict, d: str):
+    total = sum(a.nbytes for a in outputs.values())
+    assert total <= DUMP_LIMIT, f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit"
+    os.makedirs(d, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
 class ClockSampler:
     """nvidia-smi clocks / throttle reasons DURING the timed region (B200_PROFILING.md recipe)."""
 
@@ -299,8 +351,10 @@ def cpu_sample(sched: Schedule, threads: int | None = None, reps: int = 3):
     composes the step time: sum(count_i * t_i).  Every op is repeated `reps` times per thread count; the minimum is
     used, min / median are reported.  ~10-30 s of CPU work on a typical host at k=19."""
     from oracle import oracle as orc
-    try:  # a -march=native build for the host it runs on (the shipped .so is x86-64-v3)
-        so = os.path.join(ROOT, "oracle", "_build", "liboracle_native.so")
+    try:  # a -march=native build for the host it runs on (the shipped .so is x86-64-v3), outside the (possibly read-only) tree
+        tmp = tempfile.mkdtemp(prefix="h2b_oracle_")
+        atexit.register(shutil.rmtree, tmp, True)
+        so = os.path.join(tmp, "liboracle_native.so")
         subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "-s", "MARCH=native", f"OUT={so}"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
         orc._lib = None
         orc._SO = so
@@ -854,6 +908,36 @@ class Workload:
         return {"lagrange_to_coeff": ok_intt, "coeff_to_extended": ok_coset, "extended_to_coeff_roundtrip": ok_back,
                 "points_checked": len(pts) + 1}
 
+    def outputs(self) -> dict:
+        """what the last step_resident computed, as its caller receives it (for --dump-outputs):
+        commitments       every commitment of the schedule, after the all-reduce (len(msm) x 16)
+        assigned_columns  the gate columns, then the lookup columns (A + L, rows, 8)
+        coefficients      lagrange_to_coeff of each polynomial whose iNTT this rank runs (rows, 8 each)
+        extended          coeff_to_extended of each polynomial whose coset NTT this rank runs, except polynomial 0
+        extended_to_coeff extended_to_coeff of polynomial 0's coset evaluations
+        The transforms work in place on buffers that persist across steps, so these depend on warmup + steps."""
+        torch, s = self.rig.torch, self.s
+        torch.cuda.synchronize()
+
+        def rows(t, n):  # (..., n, 4) int64 on the device -> (..., dump rows, 8)
+            idx = torch.from_numpy(dump_rows(n)).to(t.device)
+            sample = t.index_select(t.dim() - 2, idx).cpu().numpy().view(np.uint64)
+            return fr_canonical(sample).reshape(*t.shape[:-2], len(idx), 8)
+
+        npoly, ext_n = s.n_poly, 1 << s.ext_k
+        to_coeff = self.my_ntt(2 * npoly) and self.my_ntt(npoly)  # ext_dev[0] holds this rank's coset NTT of polynomial 0
+        out = {"commitments": np.stack([g1_affine(c) for c in self.outs_dev.cpu().numpy().view(np.uint64)]),
+               "assigned_columns": rows(self.acols_dev, s.n) if not s.L else np.concatenate([rows(self.acols_dev, s.n), rows(self.lcols_dev, s.n)])}
+        coeffs = [rows(self.polys_dev[i], s.n) for i in sorted(self.polys_dev) if self.my_ntt(i)]
+        ext = [rows(self.ext_dev[i], ext_n) for i in sorted(self.ext_dev) if i in self.polys_dev and self.my_ntt(npoly + i) and not (i == 0 and to_coeff)]
+        if coeffs:
+            out["coefficients"] = np.stack(coeffs)
+        if ext:
+            out["extended"] = np.stack(ext)
+        if to_coeff:
+            out["extended_to_coeff"] = rows(self.ext_dev[0], ext_n)
+        return out
+
     def close(self):
         if self.side_pool:
             self.side_pool.shutdown()
@@ -874,12 +958,14 @@ def run_config(rig: Rig, sched: Schedule, steps: int, warmup: int, headline: boo
     if headline:
         res["acc"] = rig.ctx.profile_read("k_accumulate")
         res["bred"] = rig.ctx.profile_read("k_batch_affine")
+        if args.dump_outputs and rig.rank == 0:
+            write_outputs(wl.outputs(), args.dump_outputs)
     torch.cuda.synchronize()
     res["verified_resident"] = wl.verify_commitments(wl.outs_dev.cpu().numpy().view(np.uint64))
     if headline:
         # the other placement of the transforms, for the record (the rule in step_resident picks by shard size)
         dflt_overlap = wl.n_loc >= (1 << 18) or BENCH_BG_NTT > 0
-        ms_alt, _ = rig.timed(lambda: wl.step_resident(not dflt_overlap), max(1, min(steps, 5)), 1)
+        ms_alt, _ = rig.timed(lambda: wl.step_resident(not dflt_overlap), steps, 1)
         res["ms_per_step_seq"] = ms_alt if dflt_overlap else ms_step
         res["ms_per_step_ovl"] = ms_step if dflt_overlap else ms_alt
         res["transform_placement"] = "beside the commitment phases (side stream)" if dflt_overlap else "one block before the h(X) phase"
@@ -906,14 +992,14 @@ def run_b200(args):
     # host memory, commitments and evaluations come down, every column stays in HBM behind h2b_poly handles in between,
     # and the step contains the quotient / product-column / opening work create_proof does between the commitments
     wl.setup_prover()
-    ms_e2e, e2e_launches = rig.timed(wl.step_e2e_prover, max(1, min(args.steps, 10)), 2)
+    ms_e2e, e2e_launches = rig.timed(wl.step_e2e_prover, args.steps, 2)
     torch.cuda.synchronize()
     prover_check = wl.verify_prover()
     # ---- the round-1 end-to-end path for continuity: every call takes and returns HOST buffers (h2b_* without _dev)
     if os.environ.get("H2B_E2E_TRACE"):
         wl.trace = []
-    ms_e2e_ovl, _ = rig.timed(wl.step_e2e, max(1, min(args.steps, 5)), 1)
-    ms_e2e_seq, _ = rig.timed(lambda: wl.step_e2e(False), max(1, min(args.steps, 3)), 1)
+    ms_e2e_ovl, _ = rig.timed(wl.step_e2e, args.steps, 1)
+    ms_e2e_seq, _ = rig.timed(lambda: wl.step_e2e(False), args.steps, 1)
     torch.cuda.synchronize()
     verified_e2e = wl.verify_commitments(wl.outs_host)
     if wl.trace is not None and rank == 0:
@@ -1195,7 +1281,7 @@ def run_single_process(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of each step timing of the headline config")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", type=int, default=3, choices=[1, 2, 3, 4, 5], help="BASELINE.json config (1-based); 3 = ECDSA k=19 is the headline")
@@ -1204,7 +1290,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--inject-fault", default=None, choices=["skip_allreduce"], help="testing: break the multi-GPU exchange; the run must exit 3")
     ap.add_argument("--single-process", action="store_true", help="one process drives --gpus N devices through a device-group context (no torchrun)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed resident step computed to DIR/<name>.npy (float64, at most 64 MB; seeded inputs, the same on every run)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "b200" or args.single_process):
+        ap.error("--dump-outputs writes the outputs of the default GPU path (--impl b200 without --single-process)")
     args.sweep_ids = [] if args.sweep in ("none", "") else [int(x) for x in args.sweep.split(",")]
     if args.impl == "reference":
         run_reference(args)

@@ -48,6 +48,29 @@ def test_horner_mont():
     assert bench.ZETA == pyref.ZETA and bench.ROOT_OF_UNITY == pyref.ROOT_OF_UNITY
 
 
+def test_dump_outputs_are_canonical_values():
+    """--dump-outputs writes values, not representations: Montgomery limbs and Jacobian points come out as the integers
+    they stand for, in exact 32-bit limbs; the sampled rows are fixed and every schedule's dump fits the size limit"""
+    rng = np.random.default_rng(7)
+    s = rand_ints(rng, 20, pyref.R) + [0, 1, pyref.R - 1]
+    got = bench.fr_canonical(mont(s, pyref.R))
+    assert got.dtype == np.float64 and got.shape == (len(s), 8)
+    assert [sum(int(l) << (32 * i) for i, l in enumerate(row)) for row in got] == s
+    pt = pyref.g1_mul(0xfeed, pyref.G1)
+    z = 0x7654321
+    jac = ints_to_limbs([pyref.to_mont(v, pyref.P) for v in (pt[0] * z * z % pyref.P, pt[1] * z ** 3 % pyref.P, z)]).reshape(12)
+    aff = bench.g1_affine(jac)
+    assert [sum(int(l) << (32 * i) for i, l in enumerate(aff[h:h + 8])) for h in (0, 8)] == list(pt)
+    assert not bench.g1_affine(ints_to_limbs([0, pyref.to_mont(1, pyref.P), 0]).reshape(12)).any()
+    rows = bench.dump_rows(1 << 21)
+    assert len(rows) == bench.DUMP_ROWS and np.array_equal(rows, bench.dump_rows(1 << 21)) and np.all(np.diff(rows) > 0)
+    assert np.array_equal(bench.dump_rows(100), np.arange(100))
+    for cfg in (1, 2, 3, 4, 5):
+        sc = bench.Schedule(cfg)
+        arrays = sc.A + sc.L + 2 * sc.n_poly  # assigned columns, coefficients, extended + extended_to_coeff
+        assert len(sc.msm) * 16 * 8 + arrays * bench.DUMP_ROWS * 8 * 8 <= bench.DUMP_LIMIT
+
+
 def test_every_transform_has_one_owner_at_every_world_size():
     """bench.py deals whole transforms to the ranks by cost; at 8 GPUs some ranks own only a coset transform or none at
     all (the k = 14 config has 7 transforms) — every transform must still have exactly one owner"""
